@@ -14,7 +14,11 @@ followed by the path's single collective: one NCCL all-gather of the per-replica
   cpu_baseline / --impl reference: the oracle's C port of the same EM (OpenMP over panels) on the
            host cores -- the reference itself is Julia and has no Kalman/EM code (SURVEY.md 0).
 
-python bench.py --gpus N --steps K --warmup W [--impl reference]
+python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the timed path computed in its last step (rank 0) as DIR/<name>.npy, float64, so that
+two builds can be compared output for output: the inputs are the same from run to run for the same arguments.
+bench_outputs/ in the repository is ignored by git for this use.
 """
 import argparse
 import json
@@ -137,6 +141,34 @@ def host_init(Xs):
     return tuple(np.stack([i[j] for i in ini]) for j in range(4))
 
 
+DUMP_LIMIT = 60 * 2 ** 20        # array bytes written by --dump-outputs (under 64 MB with the .npy headers)
+
+
+def dump_outputs(path, per_rep, ids, shared=None):
+    """Write `shared` and `per_rep` (replication axis first; replication ids `ids`) as <path>/<name>.npy in float64, and
+    the ids as replication_id.npy.  If the total would exceed DUMP_LIMIT, a fixed seeded sample of replications is kept."""
+    shared = {n: np.asarray(a, np.float64) for n, a in (shared or {}).items()}
+    per_rep = {n: np.asarray(a, np.float64) for n, a in per_rep.items()}
+    ids = np.asarray(ids, np.float64)
+    room = DUMP_LIMIT - sum(a.nbytes for a in shared.values())
+    each = 8 + sum(a.nbytes for a in per_rep.values()) // len(ids)
+    keep = np.arange(len(ids))
+    if each * len(ids) > room:
+        keep = np.sort(np.random.default_rng(0).choice(len(ids), room // each, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for n, a in {**shared, **{n: a[keep] for n, a in per_rep.items()}, "replication_id": ids[keep]}.items():
+        np.save(os.path.join(path, n + ".npy"), a)
+
+
+def em_outputs(out, B, N, r, k, T, iters_cap, it, st):
+    """Column-major EM outputs of B panels (host arrays keyed as EmOut) -> caller-shaped arrays; log-likelihood entries
+    past each panel's iteration count are NaN (never written)."""
+    ll = out["loglik"].reshape(B, iters_cap)
+    return {"F": out["F"].reshape(B, r, T).transpose(0, 2, 1), "Lam": out["Lam"].reshape(B, r, N).transpose(0, 2, 1),
+            "R": out["R"].reshape(B, N), "A": out["A"].reshape(B, k, r).transpose(0, 2, 1), "Q": out["Q"].reshape(B, r, r).transpose(0, 2, 1),
+            "loglik": np.where(np.arange(iters_cap) < it[:, None], ll, np.nan), "iters": it, "status": st}
+
+
 CPU_SAMPLE_PANELS = 256          # the bounded CPU sample: the first 256 panels of the workload x em_iters iterations
 
 
@@ -170,7 +202,12 @@ def run_reference(args):
     if rank != 0:
         return
     iters = args.em_iters
-    cpu, t, _ = cpu_sample(iters, steps=args.steps, warmup=max(1, min(args.warmup, 2)))
+    cpu, t, out = cpu_sample(iters, steps=args.steps, warmup=max(1, min(args.warmup, 2)))
+    if args.dump_outputs:
+        ll = out["loglik"]
+        dump_outputs(args.dump_outputs, {**{n: out[n] for n in ("F", "Lam", "R", "A", "Q", "iters", "status")},
+                                         "loglik": np.where(np.arange(ll.shape[1]) < out["iters"][:, None], ll, np.nan)},
+                     np.arange(len(ll)))
     v = cpu["value"]
     print(json.dumps({"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
                       "warmup": args.warmup, "ms_per_step": 1e3 * t / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -276,6 +313,9 @@ def run_c4(args):
     ms = _timed(torch, dist, world, dev, step_device, K_)
     launches = lib.launches - l0
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:                            # records [variable, horizon, shock], as replicate.bootstrap_irf
+        dump_outputs(args.dump_outputs, {"irf": dirf.cpu().numpy().reshape(B, r, H, r).transpose(0, 3, 2, 1)}, rank * B + np.arange(B),
+                     shared={"bands": dband.cpu().numpy().reshape(len(qs), r, H, r).transpose(0, 3, 2, 1), "percentiles": qs})
     value = world * B * K_ / (ms * 1e-3)
     nfail = int(torch.isnan(dirf.view(B, -1)).any(1).sum().item())
 
@@ -376,6 +416,9 @@ def run_single_panel(args):
     ms = _timed(torch, dist, world, dev, step_device, K_)
     launches = lib.launches - l0
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, em_outputs({n: t.cpu().numpy() for n, t in dout.items()}, 1, N, r, k, T, mi,
+                                                   dit.cpu().numpy(), dst.cpu().numpy()), [rank])
     iters = int(dit.item())
     value = world * iters * K_ / (ms * 1e-3)
     hX = dX.cpu().pin_memory()
@@ -448,7 +491,10 @@ def main():
     ap.add_argument("--config", default="c5", choices=["c5", "c4", "c3", "c2-single"],
                     help="c5 (default, the headline metric): Monte-Carlo shard of C2-shaped panels; c4: bootstrap IRF bands of the "
                          "hom_fac_1 model; c3: one large panel N=2000 r=20 T=2000; c2-single: one C2 panel, EM to convergence")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if args.config != "c5":
@@ -532,6 +578,9 @@ def main():
     ms_dev, ms_wall = timed(step_device, K_)
     launches = lib.launches - l0
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:                            # later legs overwrite these buffers
+        dump_outputs(args.dump_outputs, em_outputs({n: t.cpu().numpy() for n, t in dout.items()}, B, NS, R_, k, T_, iters,
+                                                   dit.cpu().numpy(), dst.cpu().numpy()), rank * B + np.arange(B))
     ms = max(ms_dev, 0.0)
     # library work is on its own stream: the step ends with lib.sync(), so torch-stream events bracket
     # host-synchronised steps; use the larger of event / wall clock (they agree to < 1%)
